@@ -207,6 +207,30 @@ def run_reference(args, rank, world):
     print(json.dumps(line))
 
 
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, reps, engines, suffix=""):
+    """What the last timed step handed its caller, per filter of this rank: the batch update's report and the corrected filter
+    state, stacked over the filters as DIR/<name><suffix>.npy (integers as float64, the filter's own precision otherwise).
+    The inputs are seeded, so two builds run with the same arguments can be compared file by file.  Filters past the
+    64 MB budget are left out (the first ones are kept, the same ones in every run)."""
+    fields = {k: [r[k] for r in reps] for k in ("m", "rank", "cm_ok", "tri_ok", "valid", "accepted", "gamma", "p_f_G")}
+    states = [e.state() for e in engines]
+    fields["imu_state"] = [s[0] for s in states]
+    fields["clone_poses"] = [s[1] for s in states]
+    fields["covariance"] = [e.covariance() for e in engines]
+    fields["delta_x"] = [e.delta_x() for e in engines]
+    per_filter = sum(8 * np.asarray(v[0]).size for v in fields.values())
+    keep = max(1, min(len(engines), DUMP_LIMIT_BYTES // per_filter))
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, vals in fields.items():
+        a = np.stack([np.asarray(v) for v in vals[:keep]])
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        np.save(out / f"{name}{suffix}.npy", a)
+
+
 def kernel_table(obj, step_fn, reps=5):
     """per-kernel device times (CUDA events between the kernels: engine option 1, plain launches on one stream)"""
     per = {}
@@ -360,7 +384,10 @@ def main():
     ap.add_argument("--filters", type=int, default=FILTERS_PER_GPU, help="independent filters per GPU in the device batch")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--skip-extras", action="store_true", help="profiling aid: only the device-timed steps (use under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -405,13 +432,13 @@ def main():
         for w, t in zip(work, tmpl_eng):
             w.copy_state_from(t)
 
-    def device_step():
+    def device_step(full_report=False):
         restore()
         grp.stage(capi.MARGINALIZE, batches, threads=host_threads)
         work[0].synchronize()
         flush_l2()
         ms = grp.launch_timed()
-        reps = grp.fetch(batches)
+        reps = grp.fetch(batches, full=full_report)
         return ms, reps
 
     def e2e_step():
@@ -431,13 +458,15 @@ def main():
     l0 = grp.launch_count()
     t_wall0 = time.perf_counter()
     times = []
-    for _ in range(K):
-        ms, reps = device_step()
+    for k in range(K):
+        ms, reps = device_step(full_report=args.dump_outputs is not None and k == K - 1)
         times.append(ms)
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches_timed = grp.launch_count() - l0
     assert all(r["m"] == N_FEAT * (2 * N_CLONES - 3) for r in reps), [r["m"] for r in reps]
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, reps, work, suffix=f"_rank{rank}" if world > 1 else "")
     dev_ms = float(np.sum(times))
     if args.skip_extras:
         sampler.stop_flag = True

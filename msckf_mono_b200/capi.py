@@ -103,17 +103,23 @@ class Batch:
         check(lib().msckf_b200_batch_launch_timed(self.h, C.byref(ms)), "msckf_b200_batch_launch_timed")
         return ms.value
 
-    def fetch(self, batches=None):
+    def fetch(self, batches=None, full=False):
+        """per-engine reports: m, rank, accepted; `full` adds every other per-track field of msckf_b200_report"""
         batches = batches or self._keep
         n = len(self.engines)
         reps = (Report * n)()
-        accs = []
+        bufs = []
         for i, b in enumerate(batches):
-            acc = np.zeros(max(b.n_tracks, 1), dtype=np.int32)
-            reps[i].accepted = acc.ctypes.data_as(C.POINTER(C.c_int))
-            accs.append(acc)
+            nt, dt = max(b.n_tracks, 1), self.engines[i].dtype
+            buf = {"accepted": np.zeros(nt, dtype=np.int32)}
+            if full:
+                buf.update(cm_ok=np.zeros(nt, dtype=np.int32), tri_ok=np.zeros(nt, dtype=np.int32), valid=np.zeros(nt, dtype=np.int32),
+                           gamma=np.zeros(nt, dtype=dt), p_f_G=np.zeros((nt, 3), dtype=dt))
+            for k, a in buf.items():
+                setattr(reps[i], k, a.ctypes.data_as(C.POINTER(C.c_int) if a.dtype == np.int32 else C.c_void_p))
+            bufs.append(buf)
         check(lib().msckf_b200_batch_fetch(self.h, reps), "msckf_b200_batch_fetch")
-        return [{"m": reps[i].m, "rank": reps[i].rank, "accepted": accs[i][:batches[i].n_tracks]} for i in range(n)]
+        return [{"m": reps[i].m, "rank": reps[i].rank, **{k: a[:batches[i].n_tracks] for k, a in bufs[i].items()}} for i in range(n)]
 
     def update(self, mode, batches, threads=1):
         """host buffers in, reports out: packing + one H2D + kernels + one D2H (the batch's end-to-end call)."""
@@ -245,6 +251,13 @@ class Engine:
         out = np.zeros((n, n), dtype=self.dtype)
         check(lib().msckf_b200_get_covariance(self.h, out.ctypes.data_as(C.c_void_p)), "msckf_b200_get_covariance")
         return out
+
+    def state(self):
+        """(IMU state: the 29 scalars of msckf_b200_get_state, clone poses [M, 7]: p, q)"""
+        imu = np.zeros(29, dtype=self.dtype)
+        poses = np.zeros((self.num_clones(), 7), dtype=self.dtype)
+        check(lib().msckf_b200_get_state(self.h, imu.ctypes.data_as(C.c_void_p), poses.ctypes.data_as(C.c_void_p)), "msckf_b200_get_state")
+        return imu, poses
 
     def set_covariance(self, P):
         P = np.ascontiguousarray(P, dtype=self.dtype)

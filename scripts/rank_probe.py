@@ -1,6 +1,7 @@
 import sys
+from pathlib import Path
 import numpy as np
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
 from msckf_mono_b200 import capi, synth
 from tests.parity_cases import make_engine
 wl = synth.make_window_workload(n_features=300, n_clones=30, seq=0)

@@ -58,9 +58,9 @@ def test_timestamps_are_ordered_and_imu_precedes_its_frame(mav0):
     assert set(tr[:, 0].astype(np.int64)) <= set(cam_t)
 
 
-def test_player_rejects_missing_folder(engine_lib):
+def test_player_rejects_missing_folder(engine_lib, tmp_path):
     with pytest.raises(RuntimeError):
-        asl.run_player("/nonexistent/mav0", dry_run=True)
+        asl.run_player(str(tmp_path / "missing" / "mav0"), dry_run=True)
 
 
 def test_player_call_sequence_on_cpu_against_the_oracle(mav0, oracle_lib, tmp_path):
